@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the GGNN propagation step (BASELINE.json metric: node-state-updates/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of ``compute_final_node_representations`` over one batch of synthetic molecules.
 Default workload = BASELINE.json configs[1] ("cfg2": sparse GGNN, hidden=100, 4 edge types, 4 timesteps,
@@ -18,14 +18,19 @@ Default workload = BASELINE.json configs[1] ("cfg2": sparse GGNN, hidden=100, 4 
 * ``readout``    : the fused gated-regression readout against the same op sequence as torch kernels (SURVEY 8f-1).
 * ``roofline``   : algorithmic bytes of the dominant kernel / its CUDA-event duration vs the measured HBM peak.
 * ``cpu_baseline``: the fp32 PyTorch-CPU restatement of the TF1 graph (oracle/; TF 1.3 is not installable)
-                   on this box's host cores, bounded sample (rank 0, N=1 only).
+                   on the host cores, ``--steps`` timed forwards at the fastest thread count (rank 0, N=1 only).
 * ``configs``    : the other BASELINE.json configurations in the same run -- cfg1_true_default, cfg3_dense, cfg5_rgcn (per-rank shards /
-                   replicas) and cfg4 STRONG-scaled (its 1024 molecules split over the N GPUs): value, ms_per_step, roofline, e2e each.
+                   replicas) and cfg4 STRONG-scaled (its 1024 molecules split over the N GPUs): value, ms_per_step, roofline, e2e each,
+                   ``--steps`` timed steps each.
 * ``train_step_dp``: one data-parallel TRAINING step of the default workload: forward (states saved) + fused readout + backward into views
                    of one persistent flat buffer + THE one all-reduce (NCCL) + per-variable clip + Adam, all inside the CUDA-event region;
                    the all-reduce's own time and payload are reported separately, and the reduced gradient is checked against the union
                    batch of all ranks' shards computed on one GPU in the same run.
 ``--impl reference`` times that CPU restatement alone (the reference arm), with the sampling of ``cpu_baseline`` and the same ``config``.
+
+``--dump-outputs DIR`` writes the node representations of the last timed forward, [V, D] float32, one file per rank:
+``DIR/final_node_representations_rank<r>.npy`` (rank r's own shard; 64 MiB in all, a seeded row sample above that).  The reference arm
+computes rank 0's workload and writes ``..._rank0.npy``, so both arms and any two builds compare file for file.
 """
 import argparse
 import json
@@ -55,7 +60,27 @@ def parse_args():
     ap.add_argument("--no-flush", action="store_true", help="do not flush L2 between timed steps")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the `configs` block (the other BASELINE configurations)")
     ap.add_argument("--no-train-step", action="store_true", help="skip the data-parallel training step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the node representations the last timed forward computed to "
+                         "DIR/final_node_representations_rank<r>.npy, one file per rank")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024   # all ranks' files together
+
+
+def dump_output(directory, rank, a, limit):
+    """Write ``a`` ([rows, ...]) as ``directory/final_node_representations_rank<rank>.npy`` in float32.  Above ``limit`` bytes it is cut to
+    a seeded sample of its rows, the same rows for the same shape, so that dumps of two builds compare row for row."""
+    os.makedirs(directory, exist_ok=True)
+    a = np.ascontiguousarray(a, dtype=np.float32)
+    if a.nbytes > limit:
+        rows = limit // (a.nbytes // a.shape[0])
+        a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], size=rows, replace=False))]
+    np.save(os.path.join(directory, "final_node_representations_rank%d.npy" % rank), a)
 
 
 def oracle_weights(w):
@@ -70,11 +95,35 @@ def oracle_weights(w):
     return out
 
 
-def time_cpu_reference(w, budget_s=12.0, max_iters=200, threads=None):
+def pick_threads(fn, ncpu, forwards=5):
+    """The torch thread count that runs ``fn`` fastest among 1, 16, 32 and all cores: the median of ``forwards`` forwards after a short
+    warm-up, none of them part of a reported time.  The TF graph's matmuls are small, so more threads are not always faster; a setting
+    whose first forward is 50x slower than the best so far is dropped at once (all cores of a big host: seconds per forward)."""
+    import torch
+    best, tried = None, []
+    for nt in sorted({1, min(16, ncpu), min(32, ncpu), ncpu}):
+        torch.set_num_threads(nt)
+        t0 = time.perf_counter(); fn(); first = time.perf_counter() - t0
+        if best is not None and first > 50 * best[0]:
+            tried.append("%d thr: %.0f ms (one forward, skipped)" % (nt, first * 1e3))
+            continue
+        t_warm, n_warm = time.perf_counter(), 1
+        while n_warm < 2 or (n_warm < 20 and time.perf_counter() - t_warm < 0.5):   # thread pool, allocator and caches warm
+            fn(); n_warm += 1
+        times = []
+        for _ in range(forwards):
+            t0 = time.perf_counter(); fn(); times.append(time.perf_counter() - t0)
+        med = statistics.median(times)
+        tried.append("%d thr: %.2f ms" % (nt, med * 1e3))
+        if best is None or med < best[0]:
+            best = (med, nt)
+    return best[1], tried
+
+
+def time_cpu_reference(w, steps, warmup):
     """node-updates/s of the fp32 torch-CPU restatement (oracle.ggnn_oracle.sparse_propagation_torch /
-    dense_propagation_torch) on the host cores, bounded by ``budget_s`` seconds of work.  The TF graph's matmuls are
-    small, so more threads are not always faster: 1 thread, 16 threads and all cores are each timed on a slice of the
-    budget and the FASTEST setting is reported (``cores`` = the thread count that won)."""
+    dense_propagation_torch) on the host cores: at the thread count ``pick_threads`` chose, ``warmup`` untimed forwards,
+    then exactly ``steps`` timed ones, median.  ``output`` is what the last timed forward computed, [V, D]."""
     import torch
     from oracle import ggnn_oracle as O
     ow = oracle_weights(w)
@@ -92,29 +141,20 @@ def time_cpu_reference(w, budget_s=12.0, max_iters=200, threads=None):
         tw = [{k: torch.from_numpy(np.ascontiguousarray(v)) for k, v in lw.items()} for lw in ow]
         fn = lambda: O.sparse_propagation_torch(h0, adj, indeg, tw, w["engine_params"])
     ncpu = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)   # the cores this process may use
-    candidates = [threads] if threads else sorted({1, min(16, ncpu), min(32, ncpu), ncpu})
-    best, tried = None, []
     with torch.no_grad():
-        for nt in candidates:
-            torch.set_num_threads(nt)
-            t0 = time.perf_counter(); fn(); first = time.perf_counter() - t0
-            if best is not None and first > 50 * best[0]:   # hopeless setting (all cores of a big host: seconds per forward): do not spend the budget on it
-                tried.append("%d thr: %.0f ms (one forward, skipped)" % (nt, first * 1e3))
-                continue
-            t_warm, n_warm = time.perf_counter(), 1
-            while n_warm < 2 or (n_warm < 20 and time.perf_counter() - t_warm < 0.5):   # thread pool, allocator and caches warm in both arms alike
-                fn(); n_warm += 1
-            times, t_start = [], time.perf_counter()
-            while len(times) < max_iters and (time.perf_counter() - t_start) < budget_s / len(candidates):
-                t0 = time.perf_counter(); fn(); times.append(time.perf_counter() - t0)
-            med = statistics.median(times)
-            tried.append("%d thr: %.2f ms" % (nt, med * 1e3))
-            if best is None or med < best[0]:
-                best = (med, nt, len(times), sum(times))
-    med, nt, cnt, tot = best
+        nt, tried = pick_threads(fn, ncpu)
+        torch.set_num_threads(nt)
+        for _ in range(warmup):
+            fn()
+        times = []
+        for _ in range(steps):
+            t0 = time.perf_counter(); last = fn(); times.append(time.perf_counter() - t0)
+    med = statistics.median(times)
     return {"value": w["node_updates"] / med, "unit": "node-updates/s", "cores": int(nt), "kind": "port", "ms_per_step": med * 1e3,
-            "sample": "%d full forwards of %s (V=%d, M=%d) in %.1f s, median, best thread count of [%s] on a %d-core host; fp32 PyTorch-CPU "
-                      "restatement of the TF1 graph (TF 1.3 not installable)" % (cnt, w["name"], w["V"], w["M"], tot, "; ".join(tried), ncpu)}
+            "output": last.reshape(w["V"], -1).numpy(),
+            "sample": "%d timed forwards of %s (V=%d, M=%d) after %d warm-up, median, in %.1f s at %d threads (untimed choice among [%s]) on a "
+                      "%d-core host; fp32 PyTorch-CPU restatement of the TF1 graph (TF 1.3 not installable)"
+                      % (steps, w["name"], w["V"], w["M"], warmup, sum(times), nt, "; ".join(tried), ncpu)}
 
 
 class ClockSampler:
@@ -205,10 +245,10 @@ def _numa_nodes():
 def run_reference(args, rank, world):
     """Reference arm: the reference's own CPU implementation of the path.  TF 1.3 cannot be installed (no
     wheel, no network), so this is the oracle port (oracle/ggnn_oracle.py) on the host threads, sampled exactly like the
-    product arm's ``cpu_baseline`` leg (same warm-up, same iteration bound, best thread count).
+    product arm's ``cpu_baseline`` leg (same warm-up, same number of timed steps, best thread count).
     On a multi-socket host the arm is measured twice, in fresh child processes -- threads free to run on every allowed core, and threads
-    confined to NUMA node 0 (the graph's small matmuls suffer from cross-socket traffic; round 2 saw a fresh process 3x slower than the
-    product arm's in-process ``cpu_baseline`` on the same box) -- and the FASTER placement is the one reported."""
+    confined to NUMA node 0 (the graph's small matmuls suffer from cross-socket traffic; a fresh process was seen 3x slower than the
+    product arm's in-process ``cpu_baseline`` on the same machine) -- and the FASTER placement is the one reported, and dumped."""
     if rank != 0:
         return
     if os.environ.get("GGNN_REF_CHILD") != "1":
@@ -216,31 +256,42 @@ def run_reference(args, rank, world):
         allowed = os.sched_getaffinity(0) if hasattr(os, "sched_getaffinity") else set()
         node0 = sorted(nodes[0] & allowed) if len(nodes) > 1 else []
         if len(node0) >= 2 and len(node0) < len(allowed):
+            import shutil
             import subprocess
+            import tempfile
             results = []
-            for label, cpus in (("threads on all %d allowed cores" % len(allowed), None), ("threads confined to NUMA node 0 (%d cores)" % len(node0), node0)):
-                env = dict(os.environ, GGNN_REF_CHILD="1")
-                if cpus is not None:
-                    env["GGNN_REF_AFFINITY"] = ",".join(str(c) for c in cpus)
-                r = subprocess.run([sys.executable, os.path.abspath(__file__)] + sys.argv[1:], capture_output=True, text=True, env=env)
-                try:
-                    line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
-                    results.append((line["value"], label, line))
-                except Exception:   # noqa: BLE001 -- a failed placement is reported, not fatal
-                    sys.stderr.write("reference arm, %s: child failed\n%s\n" % (label, r.stderr[-1500:]))
-            if results:
-                results.sort(key=lambda t: -t[0])
-                best = results[0][2]
-                note = "; placements tried: " + " | ".join("%s: %.3g node-updates/s" % (lab, val) for val, lab, _ in results)
-                best["cpu_baseline"]["sample"] += note
-                print(json.dumps(best))
-                return
+            with tempfile.TemporaryDirectory() as tmp:
+                for i, (label, cpus) in enumerate((("threads on all %d allowed cores" % len(allowed), None),
+                                                   ("threads confined to NUMA node 0 (%d cores)" % len(node0), node0))):
+                    env = dict(os.environ, GGNN_REF_CHILD="1")
+                    if cpus is not None:
+                        env["GGNN_REF_AFFINITY"] = ",".join(str(c) for c in cpus)
+                    dump = os.path.join(tmp, str(i))   # each child dumps apart; the reported one's file is kept
+                    extra = ["--dump-outputs", dump] if args.dump_outputs else []   # the last occurrence of an option wins
+                    r = subprocess.run([sys.executable, os.path.abspath(__file__)] + sys.argv[1:] + extra, capture_output=True, text=True, env=env)
+                    try:
+                        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+                        results.append((line["value"], label, line, dump))
+                    except Exception:   # noqa: BLE001 -- a failed placement is reported, not fatal
+                        sys.stderr.write("reference arm, %s: child failed\n%s\n" % (label, r.stderr[-1500:]))
+                if results:
+                    results.sort(key=lambda t: -t[0])
+                    best = results[0][2]
+                    note = "; placements tried: " + " | ".join("%s: %.3g node-updates/s" % (lab, val) for val, lab, _, _ in results)
+                    best["cpu_baseline"]["sample"] += note
+                    if args.dump_outputs:
+                        os.makedirs(args.dump_outputs, exist_ok=True)
+                        shutil.copy(os.path.join(results[0][3], "final_node_representations_rank0.npy"), args.dump_outputs)
+                    print(json.dumps(best))
+                    return
     aff = os.environ.get("GGNN_REF_AFFINITY")
     if aff and hasattr(os, "sched_setaffinity"):
         os.sched_setaffinity(0, _parse_cpulist(aff))   # before torch creates its thread pool: the workers inherit it
     from gated_graph_neural_network_samples_b200 import workloads
     w = workloads.build(args.config, seed=0)
-    res = time_cpu_reference(w, budget_s=12.0)
+    res = time_cpu_reference(w, args.steps, args.warmup)
+    if args.dump_outputs:   # rank 0's workload: compares with the product arm's ..._rank0.npy
+        dump_output(args.dump_outputs, 0, res["output"], DUMP_LIMIT_BYTES)
     line = {"impl": "reference", "metric": "GGNN node-state-updates/sec (propagation step)", "value": res["value"],
             "unit": "node-updates/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -400,7 +451,7 @@ class Bench:
                "roofline": self.roofline(w, ms, launches / steps),
                "e2e": {"value": units / (e2e_total / steps * 1e-3), "unit": "node-updates/s", "ms_per_step": e2e_total / steps,
                        "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
-               "config": config_of(w, self.world, "strong" if strong else "weak"), "plan": eng.plan}
+               "config": config_of(w, self.world, "strong" if strong else "weak"), "plan": eng.plan, "steps": steps}
         if strong:   # the roofline of a strong-scaled batch is quoted on the WHOLE batch's bytes over the max-over-ranks time
             alg_total = self.reduce([], [float(workloads.algorithmic_bytes(w))])[1][0]
             ach = alg_total / (ms * 1e-3) / 1e9
@@ -552,6 +603,8 @@ def main():
     dev_ms_total, launches, hot_ms = B.time_forward(eng, h0, out, args.steps, args.warmup)
     wall = time.perf_counter() - wall0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:   # now: the legs below rerun the forward, and the training step updates the weights
+        dump_output(args.dump_outputs, rank, out.cpu().numpy(), DUMP_LIMIT_BYTES // world)
 
     # ---- end-to-end through the host-buffer API (pinned host inputs, H2D + D2H inside the timed region)
     e2e_ms_total, h2d, d2h, (h0_host, out_host) = B.time_e2e(eng, w, out, args.steps, args.warmup)
@@ -709,7 +762,7 @@ def main():
     others = {}
     if args.config == "cfg2" and not args.no_other_configs:
         for name in ("cfg1_true_default", "cfg3_dense", "cfg4", "cfg5_rgcn"):
-            others[name] = B.other_config(name, min(args.steps, 20))
+            others[name] = B.other_config(name, args.steps)
 
     # ---- max over ranks
     (dev_ms_total, e2e_ms_total, hot_ms, pipe_ms_total, train_ms_total, e2e_ro_max, prod_ms_max), (total_units_per_step,) = B.reduce(
@@ -760,7 +813,7 @@ def main():
             "clocks": clocks,
         }
         if not args.no_cpu_baseline and world == 1:
-            cb = time_cpu_reference(w, budget_s=12.0)
+            cb = time_cpu_reference(w, args.steps, args.warmup)
             line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")}
         print(json.dumps(line))
     if world > 1:
