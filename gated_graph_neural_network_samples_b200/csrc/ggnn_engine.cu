@@ -361,7 +361,7 @@ static int ggnn_backward_impl(ggnn_engine* e, const float* d_h_out, const ggnn_l
                               float* d_h0, ggnn_stream_t stream) {
     using namespace ggnn::bwd;
     if (!e->graph_set || !e->weights_set) return e->fail(GGNN_ESTATE, "no graph / weights set");
-    if (!e->saved_valid) return e->fail(GGNN_ESTATE, "ggnn_backward needs a preceding ggnn_forward with save_for_backward enabled");
+    if (!e->saved_valid) return e->fail(GGNN_ESTATE, "ggnn_backward needs a preceding ggnn_forward with save_for_backward enabled, and no ggnn_set_weights or new graph since");
     if (!e->has_transpose) return e->fail(GGNN_ESTATE, "enable save_for_backward BEFORE ggnn_set_graph_sparse (the source-keyed CSR is built there)");
     if (!grads || num_layers != e->L || (!d_h_out && e->V > 0)) return e->fail(GGNN_EINVAL, "bad backward arguments");
     for (int l = 0; l < e->L; ++l) {   // the weight-gradient kernels use 16-byte vector atomics
@@ -646,6 +646,8 @@ int ggnn_destroy(ggnn_engine* e) {
 
 int ggnn_set_weights(ggnn_engine* e, const ggnn_layer_weights* layers, int32_t num_layers) {
     if (!e) return GGNN_EINVAL;
+    // the saved activations belong to the weights they were computed with: a backward after new weights would mix the two
+    e->saved_valid = false;
     if (!layers || num_layers != e->L) return e->fail(GGNN_EINVAL, "expected %d layers of weights, got %d", e->L, num_layers);
     for (int l = 0; l < e->L; ++l) {
         const ggnn_layer_weights& w = layers[l];
@@ -1910,11 +1912,14 @@ int ggnn_forward(ggnn_engine* e, const float* h0, float* h_out, ggnn_stream_t st
     cudaStream_t st = (cudaStream_t)stream;
     e->last_launches = 0;
     e->last_h0 = h0; e->last_out = h_out; e->saved_valid = false;
-    if (e->V == 0) return GGNN_OK;
+    // an empty batch or a model without timesteps saves nothing, but ggnn_backward must still accept it (d_h0 = d_h_out)
+    auto mark_saved = [e]() { if (e->save) { e->saved_valid = true; e->saved_drop_keep = e->drop_keep; e->saved_drop_seed = e->drop_seed; } };
+    if (e->V == 0) { mark_saved(); return GGNN_OK; }
     if (e->save) { int rc = reserve_states(e); if (rc) return rc; }
     const size_t vd_bytes = (size_t)e->V * e->D * sizeof(float);
     if (e->total_steps == 0) {  // no propagation at all: result is the input (sparse:152 with empty loops)
         if (h_out != h0) CU_TRY(e, cudaMemcpyAsync(h_out, h0, vd_bytes, cudaMemcpyDeviceToDevice, st));
+        mark_saved();
         return GGNN_OK;
     }
     if (e->precision != GGNN_PREC_FP32) return e->stream ? forward_stream(e, h0, h_out, st) : forward_tc(e, h0, h_out, st);

@@ -394,12 +394,34 @@ class PropagationEngine:
     def set_save_for_backward(self, enable: bool):
         self._check(self.lib.ggnn_set_save_for_backward(self._h, int(bool(enable))))
 
+    def _check_grad_buffer(self, t, n: int, what: str):
+        """The library adds to gradient buffers with fp32 atomics and trusts their size: check dtype, device, layout and size here."""
+        import torch
+        if not (isinstance(t, torch.Tensor) and t.is_cuda and t.device.index == self.device and t.dtype == torch.float32
+                and t.is_contiguous()):
+            raise GgnnError("%s must be a contiguous fp32 tensor on cuda:%d" % (what, self.device))
+        if t.numel() != n:
+            raise GgnnError("%s has %d elements, expected %d" % (what, t.numel(), n))
+
     def backward(self, d_out, grads: Sequence[dict], d_h0=None):
+        """ggnn_backward: ``grads[l][field]`` are ADDED to (None skips a gradient), ``d_h0`` is overwritten.  Every buffer is checked
+        against ``weight_shapes`` / ``[V, D]`` first; fields the model does not have are ignored, as in ``set_weights``."""
+        if len(grads) != self.L:
+            raise GgnnError("expected %d layers of gradients, got %d" % (self.L, len(grads)))
+        vd = self.V * self.D
+        self._check_grad_buffer(d_out, vd, "d_out")
+        if d_h0 is not None:
+            self._check_grad_buffer(d_h0, vd, "d_h0")
         arr = (_lib.GgnnLayerGrads * len(grads))()
         for l, g in enumerate(grads):
+            shapes = weight_shapes(self.params, self.T, l)
             for f in WEIGHT_FIELDS:
                 t = g.get(f)
-                setattr(arr[l], f, None if t is None else t.data_ptr())
+                if t is None or f not in shapes:
+                    setattr(arr[l], f, None)
+                    continue
+                self._check_grad_buffer(t, int(np.prod(shapes[f])), "layer %d gradient %s" % (l, f))
+                setattr(arr[l], f, t.data_ptr())
         self._check(self.lib.ggnn_backward(self._h, d_out.data_ptr(), arr, len(grads),
                                            None if d_h0 is None else d_h0.data_ptr(), self._stream()))
 

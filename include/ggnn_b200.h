@@ -223,8 +223,10 @@ int ggnn_set_state_dropout(ggnn_engine* e, float keep_prob, uint64_t seed);
 int ggnn_state_dropout_mask(int32_t V, int32_t D, int32_t global_step, float keep_prob, uint64_t seed, uint8_t* mask_out);
 
 /* Gradient of the propagation (what optimizer.compute_gradients builds, chem_tensorflow.py:184).
- * Must follow a ggnn_forward on the same graph with save_for_backward enabled.
- * d_h_out: DEVICE [V, D]; grads: per layer, accumulated into; d_h0: DEVICE [V, D] or NULL. */
+ * Must follow a ggnn_forward on the same graph and weights with save_for_backward enabled: ggnn_set_weights or a new graph in
+ * between returns GGNN_ESTATE.  An empty batch or a model without timesteps is accepted (d_h0 = d_h_out, weight gradients untouched).
+ * d_h_out: DEVICE [V, D]; grads: per layer, each pointer NULL or ADDED to (fp32 atomics: the caller zeroes them, and two backward
+ * calls on one forward add the gradient twice); d_h0: DEVICE [V, D], OVERWRITTEN with the gradient, or NULL. */
 int ggnn_set_save_for_backward(ggnn_engine* e, int32_t enable);
 int ggnn_backward(ggnn_engine* e, const float* d_h_out, const ggnn_layer_grads* grads, int32_t num_layers,
                   float* d_h0, ggnn_stream_t stream);

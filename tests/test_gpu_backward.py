@@ -26,7 +26,8 @@ def _autograd_reference(params, T, w_np, adj, indeg, h0, G, state_dropout=None):
     th0 = torch.tensor(h0, dtype=torch.float64, requires_grad=True)
     out = O.sparse_propagation_torch(th0, adj, indeg, tw, params, dtype=torch.float64, state_dropout=state_dropout)
     (out * torch.tensor(G, dtype=torch.float64)).sum().backward()
-    return out.detach().numpy(), th0.grad.numpy(), [{k: v.grad.numpy() for k, v in lw.items()} for lw in tw]
+    # a layer without timesteps never uses its weights: autograd leaves their .grad unset, the gradient is zero
+    return out.detach().numpy(), th0.grad.numpy(), [{k: (np.zeros(v.shape) if v.grad is None else v.grad.numpy()) for k, v in lw.items()} for lw in tw]
 
 
 def _engine_grads(params, T, w_np, set_graph, h0, G, precision, state_dropout=None):
