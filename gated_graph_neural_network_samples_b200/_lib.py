@@ -69,6 +69,7 @@ SYMBOLS = {
     "ggnn_set_state_dropout": (C.c_int, [C.c_void_p, C.c_float, C.c_uint64]),
     "ggnn_state_dropout_mask": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_uint64, C.c_void_p]),
     "ggnn_set_save_for_backward": (C.c_int, [C.c_void_p, C.c_int32]),
+    "ggnn_set_backward_precision": (C.c_int, [C.c_void_p, C.c_int32]),
     "ggnn_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(GgnnLayerGrads), C.c_int32, C.c_void_p, C.c_void_p]),
     "ggnn_num_messages": (C.c_int, [C.c_void_p, C.POINTER(C.c_int64)]),
     "ggnn_get_csr": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

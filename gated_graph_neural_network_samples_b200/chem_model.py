@@ -56,6 +56,8 @@ class ChemModel(object):
         # against a stand-in engine (tests/test_chem_model_cpu.py)
         self.device = torch.device("cpu") if dev == "cpu" else torch.device("cuda", int(dev or 0))
         self.precision = args.get('--precision') or "fp32"
+        # arithmetic of the propagation's backward: "fp32" (default) or "bf16x3" (tensor cores, bit-reproducible gradients)
+        self.backward_precision = args.get('--backward_precision') or "fp32"
 
         self.max_num_vertices = self.num_edge_types = self.annotation_size = 0
         self.train_data, self.valid_data = (self.load_data(self.params[k], is_training_data=t)

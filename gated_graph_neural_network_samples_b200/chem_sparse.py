@@ -123,6 +123,8 @@ class SparseGGNNChemModel(ChemModel):
         self._padded_hidden = (h_dim + 3) // 4 * 4
         self.engine = PropagationEngine(dict(self.params, hidden_size=self._padded_hidden), T, device=self.device.index or 0,
                                         precision=self.precision)
+        if self.backward_precision != "fp32":
+            self.engine.set_backward_precision(self.backward_precision)
         self._propagation = _propagation_function()
         self._readout = gated_readout_function()
 

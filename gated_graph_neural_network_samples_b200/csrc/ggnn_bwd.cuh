@@ -334,13 +334,18 @@ __global__ void __launch_bounds__(256) csr_gather_all_kernel(GatherJob j0, Gathe
 //   d s_m = alpha_m (d alpha_m - sum_k alpha_k d alpha_k),   d a_t += d s_m <h[src], h[v]>,
 //   d h[v] += sum_m d s_m a_t h[src_m]   (this kernel, one warp per target),   d h[src] += d s_m a_t h[v]  (source kernel below).
 // dsa[slot] = d s_m a_t is left for the source kernel; scratch[slot] holds d alpha in between.
+// DET (the deterministic backward): instead of atomics into d_att_w, every block writes its per-type sums, added over its 8 warps in
+// warp order, to daw_part[block][T]; a fixed-order column sum (ggnn_bwd_tc.cuh) adds them to d_att_w.
+template <bool DET>
 __global__ void __launch_bounds__(256) attention_bwd_target_kernel(const int* __restrict__ row_ptr, const int* __restrict__ csr_src,
                                                                    const float* __restrict__ h, const float* __restrict__ P,
                                                                    const float* __restrict__ alpha, const float* __restrict__ att_w,
                                                                    float* __restrict__ dsa, float* __restrict__ dh, float* __restrict__ d_att_w,
-                                                                   int V, int D, int T) {
+                                                                   int V, int D, int T, float* __restrict__ daw_part) {
     __shared__ float s_daw[16];
+    __shared__ float s_dawp[DET ? 8 : 1][16];
     if (threadIdx.x < 16) s_daw[threadIdx.x] = 0.f;
+    if (DET && threadIdx.x < 8 * 16) s_dawp[threadIdx.x >> 4][threadIdx.x & 15] = 0.f;
     __syncthreads();
     const int v = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (v < V) {
@@ -380,7 +385,8 @@ __global__ void __launch_bounds__(256) attention_bwd_target_kernel(const int* __
                 __syncwarp();
                 if (lane == 0) dsa[m] = ds * aw;
             }
-            if (lane == 0 && d_att_w && daw != 0.f) atomicAdd(&s_daw[t], daw);
+            if (DET) { if (lane == 0) s_dawp[threadIdx.x >> 5][t] = daw; }
+            else if (lane == 0 && d_att_w && daw != 0.f) atomicAdd(&s_daw[t], daw);
         }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
@@ -389,7 +395,13 @@ __global__ void __launch_bounds__(256) attention_bwd_target_kernel(const int* __
         }
     }
     __syncthreads();
-    if (d_att_w && threadIdx.x < T && s_daw[threadIdx.x] != 0.f) atomicAdd(d_att_w + threadIdx.x, s_daw[threadIdx.x]);
+    if (DET) {
+        if (daw_part && threadIdx.x < T) {
+            float s = 0.f;
+            for (int w = 0; w < 8; ++w) s += s_dawp[w][threadIdx.x];
+            daw_part[(size_t)blockIdx.x * T + threadIdx.x] = s;
+        }
+    } else if (d_att_w && threadIdx.x < T && s_daw[threadIdx.x] != 0.f) atomicAdd(d_att_w + threadIdx.x, s_daw[threadIdx.x]);
 }
 // d h[s] += sum over the messages LEAVING s of dsa[target-CSR slot] * h[target]     (source-keyed CSR, one warp per source)
 __global__ void __launch_bounds__(256) attention_bwd_source_kernel(const int* __restrict__ trow, const int* __restrict__ ttgt,

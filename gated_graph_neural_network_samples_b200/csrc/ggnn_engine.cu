@@ -23,6 +23,7 @@
 #include "../../include/ggnn_b200.h"
 #include "ggnn_common.cuh"
 #include "ggnn_bwd.cuh"
+#include "ggnn_bwd_tc.cuh"
 #include "ggnn_readout.cuh"
 #include "ggnn_fwd_ffma.cuh"
 #include "ggnn_fwd_tc.cuh"
@@ -139,6 +140,7 @@ struct ggnn_engine {
     float drop_keep = 1.0f; unsigned long long drop_seed = 0;          // state dropout for the next forward
     float saved_drop_keep = 1.0f; unsigned long long saved_drop_seed = 0; // ... and what the saved forward used
     int last_launches = 0;
+    int bwd_precision = GGNN_PREC_FP32;   // arithmetic of ggnn_backward's GEMMs (ggnn_set_backward_precision), independent of `precision`
     std::vector<int> h_counts, h_diff, h_cursor;   // host scratch of the sparse-graph builder, kept between batches
     struct ggnn_prepared_graph* own_prep = nullptr;   // the prepared graph ggnn_set_graph_sparse builds and uploads from (reused every batch)
     std::string err;
@@ -386,6 +388,16 @@ static int ggnn_backward_impl(ggnn_engine* e, const float* d_h_out, const ggnn_l
     const size_t o_dstate = take(vd * (L + 1)), o_dha = take(vd), o_dhb = take(vd), o_dpc = take(vd), o_dpg = take(2 * vd);
     const size_t o_dxc = take((size_t)V * ldx_max), o_dxg = take((size_t)V * ldx_max), o_rh = take(vd), o_dxp = take(vd), o_at = take(vd * T), o_gt = take(vd * T);
     const size_t o_pall = take(e->use_att ? vd * T : 0), o_dsa = take(e->use_att ? (size_t)std::max<int64_t>(e->M, 1) : 0);
+    // bf16x3: split-reduction workspace of the weight-gradient GEMMs (the largest of their shapes) and per-block attention partials
+    const bool tcb = e->bwd_precision == GGNN_PREC_BF16X3;
+    size_t ws_floats = 0;
+    if (tcb) {
+        for (int nseg = 1; nseg <= std::max(maxres + 2, std::min(T, MAX_SEGS)); ++nseg)
+            for (int N : {D, 2 * D}) ws_floats = std::max(ws_floats, bwdtc::tn_workspace_floats(V, N, D, nseg, e->num_sms));
+        ws_floats = std::max(ws_floats, bwdtc::tn_workspace_floats(V, D, T, 1, e->num_sms));
+    }
+    const size_t o_ws = take(ws_floats), o_dawp = take(tcb && e->use_att ? (size_t)((V + 7) / 8) * T : 0);
+    const size_t o_bpart = take(tcb ? (size_t)((V + bwdtc::COLSUM_ROWS - 1) / bwdtc::COLSUM_ROWS) * 2 * D : 0);
     const size_t o_ptrs = off; off += 256;
     CU_TRY(e, e->bwd_buf.reserve(off));
     char* bb = (char*)e->bwd_buf.ptr;
@@ -393,7 +405,9 @@ static int ggnn_backward_impl(ggnn_engine* e, const float* d_h_out, const ggnn_l
     float *dha = (float*)(bb + o_dha), *dhb = (float*)(bb + o_dhb), *dpc = (float*)(bb + o_dpc), *dpg = (float*)(bb + o_dpg);
     float *dxc = (float*)(bb + o_dxc), *dxg = (float*)(bb + o_dxg), *rh = (float*)(bb + o_rh), *dxp = (float*)(bb + o_dxp);
     float *At = (float*)(bb + o_at), *Gt = (float*)(bb + o_gt), *Pall = (float*)(bb + o_pall), *dsa = (float*)(bb + o_dsa);
+    float *ws = (float*)(bb + o_ws), *dawp = (float*)(bb + o_dawp), *bpart = (float*)(bb + o_bpart);
     float** d_ptrs = (float**)(bb + o_ptrs);
+    if (tcb) CU_TRY(e, bwdtc::configure_tc_gemm());
     CU_TRY(e, cudaMemsetAsync(dstate, 0, vd * L * sizeof(float), st));
     CU_TRY(e, cudaMemcpyAsync(dstate + vd * L, d_h_out, vd * sizeof(float), cudaMemcpyDeviceToDevice, st));
     // forward values of node_states_per_layer
@@ -414,8 +428,20 @@ static int ggnn_backward_impl(ggnn_engine* e, const float* d_h_out, const ggnn_l
     const float* denom = (const float*)(g + e->off_denom);
     const long long n = (long long)vd;
     const int eb = (int)std::min<long long>((n + 255) / 256, 4096);
+    // ffma: the FFMA kernel whatever the backward precision (it sums in a fixed order too, without atomics)
     auto gemm_nt = [&](bool acc, const float* A, int lda, int a_stride, const float* B, int ldb, int b_stride, int nseg, float* C, int ldc,
-                       int M, int N, int K) {
+                       int M, int N, int K, bool ffma = false) {
+        if (tcb && !ffma) {   // tensor cores: one CTA per 128 x nc tile, the whole reduction in a fixed order
+            bwdtc::TcGemmParams p;
+            memset(&p, 0, sizeof p);
+            p.A = A; p.lda = lda; p.a_stride = a_stride; p.B = B; p.ldb = ldb; p.b_stride = b_stride; p.nseg = nseg;
+            p.C = C; p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.nc = bwdtc::pick_nc(N); p.acc = acc ? 1 : 0;
+            p.error_flag = (int*)e->err_flag.ptr;
+            dim3 grid((N + p.nc - 1) / p.nc, (M + bwdtc::BM - 1) / bwdtc::BM);
+            bwdtc::tc_gemm_kernel<bwdtc::MODE_NT><<<grid, bwdtc::NTHREADS, bwdtc::smem_bytes(p.nc), st>>>(p);
+            ++e->last_launches;
+            return;
+        }
         dim3 grid((N + NT_BN - 1) / NT_BN, (M + NT_BM - 1) / NT_BM);
         if (acc) gemm_nt_kernel<true><<<grid, 128, 0, st>>>(A, lda, a_stride, B, ldb, b_stride, nseg, C, ldc, M, N, K);
         else gemm_nt_kernel<false><<<grid, 128, 0, st>>>(A, lda, a_stride, B, ldb, b_stride, nseg, C, ldc, M, N, K);
@@ -425,6 +451,31 @@ static int ggnn_backward_impl(ggnn_engine* e, const float* d_h_out, const ggnn_l
     auto gemm_tn = [&](const SegList& segs, int nseg, bool a_vec, const float* B, int ldb, float* C, int ldc, size_t c_stride, float* bias, int M,
                        int N, int K) {
         if (!C && !bias) return;
+        if (tcb) {   // tensor cores, S node chunks -> workspace -> chunk-order reduce; no float atomics
+            if (bias) {   // its own fixed-order column sum: the same bits whether or not C is requested
+                const int nch = (M + bwdtc::COLSUM_ROWS - 1) / bwdtc::COLSUM_ROWS;
+                bwdtc::colsum_part_kernel<<<dim3((N + 255) / 256, nch), 256, 0, st>>>(B, ldb, M, N, bpart);
+                bwdtc::colsum_det_kernel<<<N, 256, 0, st>>>(bpart, N, nch, bias);
+                e->last_launches += 2;
+            }
+            if (!C) return;
+            const bwdtc::TnSplit sp = bwdtc::tn_split(M, N, K, nseg, e->num_sms);
+            bwdtc::TcGemmParams p;
+            memset(&p, 0, sizeof p);
+            p.B = B; p.ldb = ldb; p.nseg = nseg; p.segs = segs; p.C = C; p.ldc = ldc; p.c_stride = (long long)c_stride;
+            p.ws = sp.S > 1 ? ws : nullptr; p.M = M; p.N = N; p.K = K; p.nc = sp.nc; p.rows_per_chunk = sp.rows_per_chunk; p.ktiles = sp.ktiles;
+            p.error_flag = (int*)e->err_flag.ptr;
+            dim3 grid((N + sp.nc - 1) / sp.nc, nseg * sp.ktiles, sp.S);
+            bwdtc::tc_gemm_kernel<bwdtc::MODE_TN><<<grid, bwdtc::NTHREADS, bwdtc::smem_bytes(sp.nc), st>>>(p);
+            ++e->last_launches;
+            if (sp.S > 1) {
+                const long long total = (long long)nseg * K * N;
+                const int blocks = (int)std::min<long long>((total + 255) / 256, 8 * (long long)e->num_sms);
+                bwdtc::tn_reduce_kernel<<<blocks, 256, 0, st>>>(ws, sp.S, nseg, K, N, C, ldc, (long long)c_stride);
+                ++e->last_launches;
+            }
+            return;
+        }
         if (C) {
             const int kblocks = (K + 63) / 64;
             const int tiles = ((N + 63) / 64) * nseg * kblocks;
@@ -513,9 +564,18 @@ static int ggnn_backward_impl(ggnn_engine* e, const float* d_h_out, const ggnn_l
                 const float* alpha = nullptr;
                 if (e->use_att) {   // softmax backward first (it adds to dh_new), then the gathers are weighted by the probabilities
                     alpha = (const float*)e->att_buf.ptr + (size_t)(e->step_base[l] + s) * (size_t)std::max<int64_t>(e->M, 1);
-                    gemm_nt(false, dxp, D, 0, w.edge_weights, D, 0, 1, Pall, TD, V, TD, D);   // P[v, t*D+k] = <dx'[v], W_t[k, :]>
-                    attention_bwd_target_kernel<<<nodes_blocks, 256, 0, st>>>(row_ptr, csr_src, h, Pall, alpha, w.edge_type_attention_weights, dsa,
-                                                                              dh_new, gw.edge_type_attention_weights, V, D, T);
+                    // P[v, t*D+k] = <dx'[v], W_t[k, :]>.  Always fp32 FFMA: the softmax backward cancels sum_k alpha_k d alpha_k out of
+                    // d alpha, and a bf16x3 P (2^-16 relative) leaves d a_t of a type whose terms nearly cancel outside the gradient bar
+                    gemm_nt(false, dxp, D, 0, w.edge_weights, D, 0, 1, Pall, TD, V, TD, D, true);
+                    if (tcb) {   // per-block partials of d a_t, added in block order
+                        float* part = gw.edge_type_attention_weights ? dawp : nullptr;
+                        attention_bwd_target_kernel<true><<<nodes_blocks, 256, 0, st>>>(row_ptr, csr_src, h, Pall, alpha, w.edge_type_attention_weights,
+                                                                                        dsa, dh_new, gw.edge_type_attention_weights, V, D, T, part);
+                        if (part) { bwdtc::colsum_det_kernel<<<T, 256, 0, st>>>(part, T, nodes_blocks, gw.edge_type_attention_weights); ++e->last_launches; }
+                    } else {
+                        attention_bwd_target_kernel<false><<<nodes_blocks, 256, 0, st>>>(row_ptr, csr_src, h, Pall, alpha, w.edge_type_attention_weights,
+                                                                                         dsa, dh_new, gw.edge_type_attention_weights, V, D, T, nullptr);
+                    }
                     attention_bwd_source_kernel<<<nodes_blocks, 256, 0, st>>>(trow, ttgt, tslot, h, dsa, dh_new, V, D, T);
                     e->last_launches += 2;
                 }
@@ -2204,6 +2264,14 @@ int ggnn_set_save_for_backward(ggnn_engine* e, int32_t enable) {
     if (!e) return GGNN_EINVAL;
     e->save = enable != 0;
     e->saved_valid = false;
+    return GGNN_OK;
+}
+
+int ggnn_set_backward_precision(ggnn_engine* e, int32_t precision) {
+    if (!e) return GGNN_EINVAL;
+    if (precision == GGNN_PREC_BF16) return e->fail(GGNN_EUNSUPPORTED, "the backward has no single-MMA bf16 mode (use GGNN_PREC_BF16X3 or GGNN_PREC_FP32)");
+    if (precision != GGNN_PREC_FP32 && precision != GGNN_PREC_BF16X3) return e->fail(GGNN_EINVAL, "unknown backward precision %d", (int)precision);
+    e->bwd_precision = precision;   // applies to the next ggnn_backward; the saved activations stay valid
     return GGNN_OK;
 }
 

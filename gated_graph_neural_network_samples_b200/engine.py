@@ -394,8 +394,15 @@ class PropagationEngine:
     def set_save_for_backward(self, enable: bool):
         self._check(self.lib.ggnn_set_save_for_backward(self._h, int(bool(enable))))
 
+    def set_backward_precision(self, precision: str):
+        """Arithmetic of the following ``backward`` calls, independent of the forward's: ``"fp32"`` (default, FFMA with fp32 atomics) or
+        ``"bf16x3"`` (tensor cores, bf16 hi/lo split, fixed summation order: bit-reproducible gradients).  Keeps the saved activations."""
+        if precision not in PRECISIONS:
+            raise GgnnError("unknown backward precision %r (expected 'fp32' or 'bf16x3')" % (precision,))
+        self._check(self.lib.ggnn_set_backward_precision(self._h, PRECISIONS[precision]))
+
     def _check_grad_buffer(self, t, n: int, what: str):
-        """The library adds to gradient buffers with fp32 atomics and trusts their size: check dtype, device, layout and size here."""
+        """The library adds to gradient buffers and trusts their size: check dtype, device, layout and size here."""
         import torch
         if not (isinstance(t, torch.Tensor) and t.is_cuda and t.device.index == self.device and t.dtype == torch.float32
                 and t.is_contiguous()):

@@ -225,9 +225,22 @@ int ggnn_state_dropout_mask(int32_t V, int32_t D, int32_t global_step, float kee
 /* Gradient of the propagation (what optimizer.compute_gradients builds, chem_tensorflow.py:184).
  * Must follow a ggnn_forward on the same graph and weights with save_for_backward enabled: ggnn_set_weights or a new graph in
  * between returns GGNN_ESTATE.  An empty batch or a model without timesteps is accepted (d_h0 = d_h_out, weight gradients untouched).
- * d_h_out: DEVICE [V, D]; grads: per layer, each pointer NULL or ADDED to (fp32 atomics: the caller zeroes them, and two backward
- * calls on one forward add the gradient twice); d_h0: DEVICE [V, D], OVERWRITTEN with the gradient, or NULL. */
+ * d_h_out: DEVICE [V, D]; grads: per layer, each pointer NULL or ADDED to (fp32 atomics by default, a fixed order with
+ * ggnn_set_backward_precision(GGNN_PREC_BF16X3): the caller zeroes them, and two backward calls on one forward add the gradient
+ * twice); d_h0: DEVICE [V, D], OVERWRITTEN with the gradient, or NULL. */
 int ggnn_set_save_for_backward(ggnn_engine* e, int32_t enable);
+/* Arithmetic of ggnn_backward's GEMMs, independent of the forward's ggnn_config.precision (any cell, attention, the dense matrix walk,
+ * state dropout):
+ *   GGNN_PREC_FP32    the default: FFMA on CUDA cores; weight gradients are summed with fp32 atomics, so two calls on the same
+ *                     forward may differ in the last bits.
+ *   GGNN_PREC_BF16X3  tcgen05 tensor cores, every operand split into bf16 hi + lo, 3 MMAs per product accumulated in fp32 (the
+ *                     arithmetic of the bf16x3 forward).  No float atomics: every gradient element is still ADDED to the caller's buffer,
+ *                     but once and in a fixed order, so d_h0 and all weight gradients are bit-identical across calls on the same GPU
+ *                     with the same inputs, and a NULL subset of the gradients leaves the requested ones bitwise unchanged.
+ *   GGNN_PREC_BF16    GGNN_EUNSUPPORTED.  Any other value: GGNN_EINVAL.
+ * May be called at any time, also between a forward and its backward: it applies to the next ggnn_backward and keeps the saved
+ * activations valid. */
+int ggnn_set_backward_precision(ggnn_engine* e, int32_t precision);
 int ggnn_backward(ggnn_engine* e, const float* d_h_out, const ggnn_layer_grads* grads, int32_t num_layers,
                   float* d_h0, ggnn_stream_t stream);
 
